@@ -11,8 +11,11 @@ CUDA events the roofline is computed from.  `e2e` repeats the step through the H
 points (pinned host memory, H2D + D2H inside the timed region).  The CPU arm (`cpu_baseline`, `--impl
 reference`) times oracle/rs_simd.c -- the reference itself has no RS code (SURVEY.md 0.1).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) as float32 .npy files;
+the inputs depend only on the arguments, so two builds can be compared file for file.
 """
 import argparse
 import json
@@ -55,7 +58,13 @@ def parse():
     ap.add_argument("--sweep-stripes", type=int, default=4096, help="stripes per code per GPU in the sweep extra")
     ap.add_argument("--sweep-e2e-stripes", type=int, default=512,
                     help="stripes per code per GPU in the HOST-buffer (end-to-end) sweep companion")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's outputs of the last step to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     if a.blocks <= 0:
         a.blocks = 8192 if int(os.environ.get("WORLD_SIZE", "1")) >= 8 else 4096
     return a
@@ -190,6 +199,33 @@ def alg_bytes_per_pass(k, m, e, n, L):
     """ALGORITHMIC bytes (SURVEY.md 8(d)): encode reads k*L, writes m*L per stripe; reconstruct
     with e erasures reads k*L, writes e*L.  (k*L = B up to the <k bytes of tail padding.)"""
     return n * (k + m) * L, n * (k + e) * L
+
+
+DUMP_SHARD_BYTES = 56_000_000  # float32 budget of the two shard samples; with the rest the dump stays under 64 MB
+
+
+def dump_outputs(out_dir, parity, shards, present, status, k, m, n, L, stride):
+    """Write what the step's caller receives, as float32 .npy files: `encode_parity` and `reconstruct_shards`
+    (the rebuilt erased shards, in shard order) of a fixed seeded sample of stripes `sample_stripes`, each
+    shard cut to its length L (and, if one stripe alone would not fit the budget, to its first bytes), and
+    `reconstruct_status` of every stripe."""
+    import torch
+
+    s = min(n, 16, max(1, DUMP_SHARD_BYTES // (2 * m * L * 4)))
+    w = min(L, DUMP_SHARD_BYTES // (2 * m * s * 4))
+    idx = np.sort(np.random.default_rng(SEED).choice(n, s, replace=False))
+    it = torch.from_numpy(idx).to(parity.device)
+    erased = (present[torch.from_numpy(idx)] == 0).to(parity.device)
+    out = {
+        "sample_stripes": idx,
+        "encode_parity": parity.view(n, m, stride)[it, :, :w],
+        "reconstruct_shards": shards.view(n, k + m, stride)[it][erased].view(s, m, stride)[:, :, :w],
+        "reconstruct_status": status,
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else a
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 # ------------------------------------------------------------------ CPU arm (oracle port)
@@ -402,6 +438,8 @@ def run_ours(args, rank, world, local_rank):
     clk.sample_until(ev1)  # the host is ahead of the GPU: these samples fall inside the timed region
     barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, parity, shards, present, status, k, m, n, L, stride)
     # parity of the timed work: reconstructed shards == originals (per-shard blake2sums), parity unchanged
     check_results("graph-replayed timed region")
     graph_used = g_step is not None
