@@ -20,6 +20,7 @@ __all__ = ["GarageEc", "EcError", "load_library", "lib_path", "ABI_SYMBOLS",
 
 OK = 0
 E_INVALID, E_CUDA, E_NOMEM, E_UNRECOVERABLE, E_NODEVICE, E_ALIGN = -1, -2, -3, -4, -5, -6
+E_UNCORRECTABLE = -7
 VANDERMONDE, CAUCHY = 0, 1
 MEM_HOST, MEM_DEVICE = 0, 1
 MAX_K, MAX_M = 32, 8
@@ -36,6 +37,7 @@ ABI_SYMBOLS = [
     "garage_ec_encode_blocks_with_sums", "garage_ec_scrub_repair",
     "garage_ec_numa_info", "garage_ec_bind_thread", "garage_ec_debug_fail_after",
     "garage_ec_set_sum_kind", "garage_ec_set_wait_mode", "garage_ec_copy_for_dma", "garage_ec_shard_sum_host", "garage_ec_reconstruct_stripes",
+    "garage_ec_correct",
 ]
 
 
@@ -86,6 +88,7 @@ def load_library(build=True):
     L.garage_ec_encode.argtypes = [vp, vp, vp, vp, sz, sz, i32, vp]
     L.garage_ec_reconstruct.argtypes = [vp, vp, vp, vp, vp, vp, sz, sz, i32, vp]
     L.garage_ec_verify.argtypes = [vp, vp, vp, vp, sz, sz, i32, vp]
+    L.garage_ec_correct.argtypes = [vp, vp, vp, vp, vp, vp, sz, sz, i32, vp]
     L.garage_ec_encode_blocks.argtypes = [vp, vp, vp, sz, vp, sz]
     L.garage_ec_encode_blocks_with_sums.argtypes = [vp, vp, vp, sz, vp, vp, sz]
     L.garage_ec_scrub_repair.argtypes = [vp, vp, vp, vp, vp, vp, sz, sz, i32, vp]
@@ -266,6 +269,14 @@ class GarageEc:
         kind, st = self._stream(shards)
         return self._check(self._L.garage_ec_verify(self._h, _ptr(shards), _ptr(mismatch), _ptr(shard_len),
                                                     stride, n, kind, st))
+
+    def correct(self, shards, stride, n, present=None, status=None, fixed=None, shard_len=None):
+        """error-locating decode: find and repair wrong shards from the parity alone (garage_ec_correct).
+        HOST mode returns 0, E_UNRECOVERABLE or E_UNCORRECTABLE (per-stripe detail in `status`)."""
+        kind, st = self._stream(shards)
+        return self._check(self._L.garage_ec_correct(self._h, _ptr(shards), _ptr(present), _ptr(status), _ptr(fixed),
+                                                     _ptr(shard_len), stride, n, kind, st),
+                           (E_UNRECOVERABLE, E_UNCORRECTABLE))
 
     # -- per-shard integrity (blake2sum of every shard)
     def shard_sums(self, shards, sums_out, stride, n, per_stripe, shard_len=None):

@@ -1085,6 +1085,24 @@ struct garage_bm {
             int who[64];
             storage_nodes_of(h, who);
             SlotLease trial(stripe_slots);
+            // First let the parity locate the wrong shards (up to floor((m - absent) / 2) of them, where the
+            // search below finds one); a miscorrection cannot slip through, the content hash decides.
+            {
+                memcpy(trial.p, slot.p, (size_t)tot * slot_stride);
+                int32_t st = 0;
+                uint8_t fixed[GARAGE_EC_MAX_K + GARAGE_EC_MAX_M] = {0};
+                const uint32_t L = (uint32_t)shard_len_of(block_len);
+                if (garage_ec_correct(ec, trial.p, have, &st, fixed, &L, slot_stride, 1, GARAGE_EC_MEM_HOST, nullptr) ==
+                        GARAGE_EC_OK) {
+                    assemble(trial.p, block_len, out);
+                    if (content_ok(h, out, block_len)) {
+                        for (int i = 0; i < tot; i++)
+                            if (fixed[i]) quarantine(who[i], h);
+                        *out_len = block_len;
+                        return GARAGE_BM_OK;
+                    }
+                }
+            }
             for (int x = 0; x < tot; x++) {
                 if (!have[x]) continue;
                 uint8_t h2[GARAGE_EC_MAX_K + GARAGE_EC_MAX_M], w2[GARAGE_EC_MAX_K + GARAGE_EC_MAX_M] = {0};

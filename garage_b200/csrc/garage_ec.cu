@@ -98,6 +98,9 @@ struct garage_ec_ctx {
     std::vector<cudaEvent_t> free_events;
     std::atomic<uint64_t> launches{0};
     std::atomic<int> batch_copy_ok{1};  // cudaMemcpyBatchAsync usable (cleared on first failure)
+    // generalized-RS structure of P (garage_ec_correct): log of locator X_r and of column multiplier v_r
+    bool grs_ok = false;
+    uint8_t grs_logx[kMaxK + kMaxM] = {0}, grs_logv[kMaxK + kMaxM] = {0};
     char last_error[256] = {0};
 };
 
@@ -452,6 +455,76 @@ int run_reconstruct(garage_ec_ctx *ctx, uint8_t *shards, const uint8_t *present,
 
 size_t plan_scratch_bytes(size_t n) { return n * sizeof(StripePlan) + 16; }
 
+// ---- error-locating decode (garage_ec_correct) --------------------------------------------
+// scratch: mismatch[n] | list[n] | bad[n] | count | err_mask[n]
+inline size_t align16(size_t v) { return (v + 15) & ~(size_t)15; }
+size_t correct_scratch_bytes(size_t n) { return 3 * align16(n * 4) + 16 + n * 8; }
+
+template <int M>
+cudaError_t launch_correct_t(garage_ec_ctx *ctx, const CorrectParams &cp, cudaStream_t st)
+{
+    const unsigned grid = (unsigned)ctx->sm_count * 8;  // persistent: the number of listed stripes is only known on the device
+    rs_correct_scan_kernel<M><<<grid, kCorrectThreads, 0, st>>>(cp);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    rs_correct_apply_kernel<M><<<grid, kCorrectThreads, 0, st>>>(cp);
+    ctx->launches.fetch_add(2, std::memory_order_relaxed);
+    return cudaGetLastError();
+}
+
+// Device-resident correct of n stripes: check (verify kernel), list, scan, apply -- all stream ordered.
+int run_correct(garage_ec_ctx *ctx, uint8_t *shards, const uint8_t *present, int32_t *status, uint8_t *fixed,
+                const uint32_t *shard_len, size_t stride, size_t n, uint8_t *scratch, cudaStream_t st)
+{
+    const size_t tot = ctx->k + ctx->m;
+    uint32_t *mismatch = reinterpret_cast<uint32_t *>(scratch);
+    uint32_t *list = reinterpret_cast<uint32_t *>(scratch + align16(n * 4));
+    uint32_t *bad = reinterpret_cast<uint32_t *>(scratch + 2 * align16(n * 4));
+    uint32_t *count = reinterpret_cast<uint32_t *>(scratch + 3 * align16(n * 4));
+    auto *err_mask = reinterpret_cast<unsigned long long *>(scratch + 3 * align16(n * 4) + 16);
+    cudaError_t e = cudaMemsetAsync(mismatch, 0, n * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(count, 0, 4, st);
+    if (e != cudaSuccess) return set_cuda_error(ctx, e, "cudaMemsetAsync(correct scratch)");
+    int rc = run_uniform(ctx, kModeVerify, shards, tot * stride, nullptr, 0, mismatch, shard_len, stride, n, st);
+    if (rc) return rc;
+    CorrectParams cp;
+    memset(&cp, 0, sizeof(cp));
+    cp.shards = shards;
+    cp.present = present;
+    cp.shard_len = shard_len;
+    cp.mismatch = mismatch;
+    cp.status = status;
+    cp.fixed = fixed;
+    cp.list = list;
+    cp.count = count;
+    cp.err_mask = err_mask;
+    cp.bad = bad;
+    cp.stride = (uint32_t)stride;
+    cp.n = (uint32_t)n;
+    cp.k = (uint32_t)ctx->k;
+    cp.m = (uint32_t)ctx->m;
+    cp.items_per_stripe = (uint32_t)((stride + kCorrectThreads - 1) / kCorrectThreads);
+    memcpy(cp.logx, ctx->grs_logx, tot);
+    memcpy(cp.logv, ctx->grs_logv, tot);
+    rs_correct_list_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(cp);
+    ctx->launches.fetch_add(1, std::memory_order_relaxed);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return set_cuda_error(ctx, e, "rs_correct_list_kernel launch");
+    switch (ctx->m) {
+    case 1: e = launch_correct_t<1>(ctx, cp, st); break;
+    case 2: e = launch_correct_t<2>(ctx, cp, st); break;
+    case 3: e = launch_correct_t<3>(ctx, cp, st); break;
+    case 4: e = launch_correct_t<4>(ctx, cp, st); break;
+    case 5: e = launch_correct_t<5>(ctx, cp, st); break;
+    case 6: e = launch_correct_t<6>(ctx, cp, st); break;
+    case 7: e = launch_correct_t<7>(ctx, cp, st); break;
+    case 8: e = launch_correct_t<8>(ctx, cp, st); break;
+    default: e = cudaErrorInvalidConfiguration;
+    }
+    if (e != cudaSuccess) return set_cuda_error(ctx, e, "rs_correct kernels launch");
+    return GARAGE_EC_OK;
+}
+
 // ---- batched async copies ---------------------------------------------------------------
 // Reconstruct moves many shard-sized pieces per stripe (only the k survivors go up, only the
 // rebuilt shards come back).  One cudaMemcpyBatchAsync per chunk instead of thousands of
@@ -560,6 +633,14 @@ int create_common(garage_ec_ctx **out, int device, int k, int m, const uint8_t *
         delete ctx;
         return GARAGE_EC_E_INVALID;
     }
+    {
+        uint8_t v[kMaxK + kMaxM];
+        ctx->grs_ok = h_grs_multipliers(k, m, ctx->P, v);
+        for (int r = 0; ctx->grs_ok && r < k + m; r++) {
+            ctx->grs_logx[r] = h_gf_log[(uint8_t)(r ^ kLocShift)];
+            ctx->grs_logv[r] = h_gf_log[v[r]];
+        }
+    }
     ctx->sm_count = prop.multiProcessorCount;
     ctx->smem_optin = prop.sharedMemPerBlockOptin;
     if (cudaSetDevice(device) != cudaSuccess) {
@@ -606,6 +687,7 @@ const char *garage_ec_strerror(int code)
     case GARAGE_EC_E_UNRECOVERABLE: return "stripe unrecoverable: fewer than k shards present";
     case GARAGE_EC_E_NODEVICE: return "no usable sm_100 CUDA device (no CPU fallback)";
     case GARAGE_EC_E_ALIGN: return "pointer or stride not 16-byte aligned";
+    case GARAGE_EC_E_UNCORRECTABLE: return "stripe uncorrectable: a column has more wrong shards than the parity can locate";
     default: return "unknown error";
     }
 }
@@ -1123,6 +1205,124 @@ int garage_ec_reconstruct_stripes(garage_ec_ctx *ctx, uint8_t *const *stripes, c
     }
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     return reconstruct_host(ctx, nullptr, stripes, present, want, status, shard_len, stride, n_stripes);
+}
+
+// --------------------------------------------------------------------------- CORRECT
+// HOST: the present shards go up; once a chunk's status and fixed flags are on the host, exactly the
+// rebuilt (absent) and fixed shards of its corrected stripes come back -- a clean chunk downloads only
+// those two arrays.  Same per-lane Pending / finish pattern as the scrub sweep.
+static int correct_host(garage_ec_ctx *ctx, uint8_t *shards, const uint8_t *present, int32_t *status, uint8_t *fixed,
+                        const uint32_t *shard_len, size_t stride, size_t n)
+{
+    const size_t tot = ctx->k + ctx->m;
+    // declared before the lane lease: they must outlive the stream work the lease waits for
+    std::vector<int32_t> st_host(status ? 0 : n);
+    std::vector<uint8_t> fx_host(fixed ? 0 : n * tot);
+    CopyBatch up, down;
+    LEASE_LANES(ctx, lanes);
+    size_t cs = kHostChunkBytes / (tot * stride);
+    if (cs < 1) cs = 1;
+    if (cs > n) cs = n;
+    const size_t o_present = 0, o_fixed = align_up(cs * tot, 16), o_status = o_fixed + align_up(cs * tot, 16);
+    const size_t o_len = o_status + align_up(cs * 4, 16), o_scr = o_len + align_up(cs * 4, 16);
+    const size_t small = o_scr + correct_scratch_bytes(cs);
+    for (HostLane &L : lanes.set->lanes) {
+        int rc = lane_reserve(ctx, L, cs * tot * stride, small);
+        if (rc) return rc;
+    }
+    int32_t *st_out = status ? status : st_host.data();
+    uint8_t *fx_out = fixed ? fixed : fx_host.data();
+    struct Pending {
+        bool active = false;
+        size_t s0 = 0, cnt = 0;
+    } pend[kHostLanes];
+    auto finish = [&](size_t lane_i) -> int {
+        Pending &P = pend[lane_i];
+        if (!P.active) return GARAGE_EC_OK;
+        HostLane &L = lanes[lane_i];
+        CU_TRY(ctx, lane_wait(ctx, L));  // status + fixed of this chunk are on the host
+        for (size_t s = P.s0; s < P.s0 + P.cnt; s++) {
+            if (st_out[s] != 0) continue;
+            const size_t len = shard_len ? shard_len[s] : stride;
+            for (size_t i = 0; i < tot; i++)
+                if ((present && !present[s * tot + i]) || fx_out[s * tot + i])
+                    down.add(shards + (s * tot + i) * stride, L.d_buf + ((s - P.s0) * tot + i) * stride, align_up(len, 16));
+        }
+        int r = down.flush(ctx, cudaMemcpyDeviceToHost, L.stream);
+        P.active = false;
+        return r;
+    };
+    size_t c = 0;
+    for (size_t s0 = 0; s0 < n; s0 += cs, c++) {
+        const size_t lane_i = c % kHostLanes;
+        HostLane &L = lanes[lane_i];
+        int rc = finish(lane_i);
+        if (rc) return rc;
+        const size_t cnt = n - s0 < cs ? n - s0 : cs;
+        if (present) {
+            for (size_t s = s0; s < s0 + cnt; s++)
+                for (size_t i = 0; i < tot; i++)
+                    if (present[s * tot + i])
+                        up.add(L.d_buf + ((s - s0) * tot + i) * stride, shards + (s * tot + i) * stride, stride);
+            rc = up.flush(ctx, cudaMemcpyHostToDevice, L.stream);
+            if (rc) return rc;
+            CU_TRY(ctx, cudaMemcpyAsync(L.d_small + o_present, present + s0 * tot, cnt * tot, cudaMemcpyHostToDevice,
+                                        L.stream));
+        } else {
+            CU_TRY(ctx, cudaMemcpyAsync(L.d_buf, shards + s0 * tot * stride, cnt * tot * stride, cudaMemcpyHostToDevice,
+                                        L.stream));
+        }
+        const uint32_t *d_len = nullptr;
+        if (shard_len) {
+            CU_TRY(ctx, cudaMemcpyAsync(L.d_small + o_len, shard_len + s0, cnt * 4, cudaMemcpyHostToDevice, L.stream));
+            d_len = reinterpret_cast<const uint32_t *>(L.d_small + o_len);
+        }
+        rc = run_correct(ctx, L.d_buf, present ? L.d_small + o_present : nullptr,
+                         reinterpret_cast<int32_t *>(L.d_small + o_status), L.d_small + o_fixed, d_len, stride, cnt,
+                         L.d_small + o_scr, L.stream);
+        if (rc) return rc;
+        CU_TRY(ctx, cudaMemcpyAsync(st_out + s0, L.d_small + o_status, cnt * 4, cudaMemcpyDeviceToHost, L.stream));
+        CU_TRY(ctx, cudaMemcpyAsync(fx_out + s0 * tot, L.d_small + o_fixed, cnt * tot, cudaMemcpyDeviceToHost, L.stream));
+        pend[lane_i].active = true;
+        pend[lane_i].s0 = s0;
+        pend[lane_i].cnt = cnt;
+    }
+    for (size_t l = 0; l < (size_t)kHostLanes; l++) {
+        int rc = finish(l);
+        if (rc) return rc;
+    }
+    for (HostLane &L : lanes.set->lanes) CU_TRY(ctx, lane_wait(ctx, L));
+    bool unrec = false, uncorr = false;
+    for (size_t s = 0; s < n; s++) {
+        unrec |= st_out[s] == GARAGE_EC_E_UNRECOVERABLE;
+        uncorr |= st_out[s] == GARAGE_EC_E_UNCORRECTABLE;
+    }
+    return unrec ? GARAGE_EC_E_UNRECOVERABLE : (uncorr ? GARAGE_EC_E_UNCORRECTABLE : GARAGE_EC_OK);
+}
+
+int garage_ec_correct(garage_ec_ctx *ctx, uint8_t *shards, const uint8_t *present, int32_t *status, uint8_t *fixed,
+                      const uint32_t *shard_len, size_t stride, size_t n_stripes, int mem_kind, void *cuda_stream)
+{
+    if (!ctx || (mem_kind != GARAGE_EC_MEM_HOST && mem_kind != GARAGE_EC_MEM_DEVICE)) return GARAGE_EC_E_INVALID;
+    if (!ctx->grs_ok) return GARAGE_EC_E_INVALID;  // custom matrix without GRS structure: errors cannot be located
+    int rc = check_geometry(ctx, stride, n_stripes, ctx->k + ctx->m);
+    if (rc) return rc;
+    if (n_stripes == 0) return GARAGE_EC_OK;
+    if (!shards) return GARAGE_EC_E_INVALID;
+    if (!aligned16(shards)) return GARAGE_EC_E_ALIGN;
+    if (n_stripes * (size_t)(ctx->k + ctx->m) > 0xffffffffull) return GARAGE_EC_E_INVALID;
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    if (mem_kind == GARAGE_EC_MEM_HOST)
+        return correct_host(ctx, shards, present, status, fixed, shard_len, stride, n_stripes);
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    void *scratch = nullptr;
+    CU_TRY(ctx, ctx->pool ? cudaMallocFromPoolAsync(&scratch, correct_scratch_bytes(n_stripes), ctx->pool, st)
+                          : cudaMallocAsync(&scratch, correct_scratch_bytes(n_stripes), st));
+    rc = run_correct(ctx, shards, present, status, fixed, shard_len, stride, n_stripes, static_cast<uint8_t *>(scratch), st);
+    cudaError_t e = cudaFreeAsync(scratch, st);
+    if (rc) return rc;
+    if (e != cudaSuccess) return set_cuda_error(ctx, e, "cudaFreeAsync");
+    return GARAGE_EC_OK;
 }
 
 // --------------------------------------------------------------------------- SHARD SUMS

@@ -85,4 +85,61 @@ inline bool h_build_matrix(int k, int m, int kind, uint8_t *P)
     return true;
 }
 
+// Column multipliers of the generalized Reed-Solomon structure of the code [I; P] with evaluation
+// points r = 0..k+m-1: v with  sum_r v_r r^l c_r = 0  for every codeword c and l < m.  Written per
+// data column j (the codeword e_j + P[:, j]):  v_j j^l + sum_i v_{k+i} (k+i)^l P[i][j] = 0.  The
+// k*m x (k+m) system must have a one-dimensional null space with no zero entry; false otherwise
+// (a matrix that is not GRS with these points: errors cannot be located with syndromes).
+inline bool h_grs_multipliers(int k, int m, const uint8_t *P, uint8_t *v)
+{
+    const int n = k + m;
+    uint8_t A[GARAGE_EC_MAX_K_HOST * GARAGE_EC_MAX_M_HOST][GARAGE_EC_MAX_K_HOST + GARAGE_EC_MAX_M_HOST];
+    auto pw = [](uint8_t a, int e) {
+        uint8_t r = 1;
+        for (int i = 0; i < e; i++) r = h_mul(r, a);
+        return r;
+    };
+    int rows = 0;
+    for (int j = 0; j < k; j++)
+        for (int l = 0; l < m; l++, rows++) {
+            for (int c = 0; c < n; c++) A[rows][c] = 0;
+            A[rows][j] = pw((uint8_t)j, l);
+            for (int i = 0; i < m; i++) A[rows][k + i] = h_mul(pw((uint8_t)(k + i), l), P[i * k + j]);
+        }
+    // row echelon form; the null space is one-dimensional iff exactly one column has no pivot
+    int piv_of_col[GARAGE_EC_MAX_K_HOST + GARAGE_EC_MAX_M_HOST];
+    int r0 = 0, free_col = -1;
+    for (int c = 0; c < n; c++) {
+        piv_of_col[c] = -1;
+        int pr = -1;
+        for (int r = r0; r < rows; r++)
+            if (A[r][c]) { pr = r; break; }
+        if (pr < 0) {
+            if (free_col >= 0) return false;  // null space of dimension >= 2
+            free_col = c;
+            continue;
+        }
+        for (int x = 0; x < n; x++) {
+            const uint8_t t = A[r0][x];
+            A[r0][x] = A[pr][x];
+            A[pr][x] = t;
+        }
+        const uint8_t iv = h_inv(A[r0][c]);
+        for (int x = 0; x < n; x++) A[r0][x] = h_mul(A[r0][x], iv);
+        for (int r = 0; r < rows; r++) {
+            const uint8_t f = A[r][c];
+            if (r == r0 || !f) continue;
+            for (int x = 0; x < n; x++) A[r][x] ^= h_mul(f, A[r0][x]);
+        }
+        piv_of_col[c] = r0++;
+    }
+    if (free_col < 0) return false;  // only the zero vector: not a GRS code with these points
+    // reduced form: v_c = A[piv][free] * v_free for pivot columns (characteristic 2), v_free = 1
+    for (int c = 0; c < n; c++) {
+        v[c] = c == free_col ? 1 : A[piv_of_col[c]][free_col];
+        if (!v[c]) return false;
+    }
+    return true;
+}
+
 }  // namespace garage_ec

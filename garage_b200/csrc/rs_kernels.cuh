@@ -1721,4 +1721,363 @@ __global__ void __launch_bounds__(256) adler8_shards_kernel(const __grid_constan
     }
 }
 
+// ------------------------------------------------------------------ error-locating decode (garage_ec_correct)
+// Both built-in matrices (and any matrix that passes h_grs_multipliers) define a generalized RS code: the
+// parity-check rows H[l][r] = v_r X_r^l, l < m, annihilate every codeword.  Locator X_r = r xor kLocShift
+// (shifting every evaluation point by one constant keeps the code and the v_r; the shift keeps X_r != 0).
+// Pipeline (DESIGN.md section 4, "Error-locating decode"):
+//   1. check:  rs_apply_kernel<kModeVerify> -- the streaming verify, unchanged: mismatch[s] != 0 iff some
+//      column of stripe s is not a codeword;
+//   2. list:   rs_correct_list_kernel -- status / fixed of every stripe; stripes with an absent shard or a
+//      mismatch go to a compacted list (device side: no host round trip, graph-capturable);
+//   3. scan:   rs_correct_scan_kernel<M> -- every byte column of every listed stripe: GRS syndromes,
+//      errors-and-erasures decoding; writes nothing but the per-stripe union of error positions and an
+//      "uncorrectable" flag;
+//   4. apply:  rs_correct_apply_kernel<M> -- listed stripes whose every column decoded: decode again and
+//      write the erased and the wrong shards (zero padding to roundup16); the rest only get status -7.
+constexpr uint32_t kLocShift = 0x80;
+constexpr int kCorrectThreads = 256;  // one byte column per thread
+
+struct CorrectParams {
+    uint8_t *shards;              // stripe s, shard r at (s*(k+m) + r) * stride
+    const uint8_t *present;       // nullable (= all present)
+    const uint32_t *shard_len;    // nullable (= stride)
+    const uint32_t *mismatch;     // check pass result
+    int32_t *status;              // nullable
+    uint8_t *fixed;               // nullable, n*(k+m)
+    uint32_t *list;               // compacted stripe indices, list[0 .. *count)
+    uint32_t *count;
+    unsigned long long *err_mask;  // per list entry: union of the error positions of its columns
+    uint32_t *bad;                 // per list entry: != 0 if some column had more than t errors
+    uint32_t stride, n, k, m;
+    uint32_t items_per_stripe;    // ceil(stride / kCorrectThreads)
+    uint8_t logx[kMaxK + kMaxM];  // log X_r
+    uint8_t logv[kMaxK + kMaxM];  // log v_r
+};
+
+// one thread per stripe: presence, status, fixed row; stripes that need the decoder are listed
+__global__ void rs_correct_list_kernel(const __grid_constant__ CorrectParams p)
+{
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= p.n) return;
+    const uint32_t tot = p.k + p.m;
+    uint32_t absent = 0;
+    if (p.present)
+        for (uint32_t r = 0; r < tot; r++) absent += p.present[(size_t)s * tot + r] ? 0u : 1u;
+    if (p.fixed)
+        for (uint32_t r = 0; r < tot; r++) p.fixed[(size_t)s * tot + r] = 0;
+    if (absent > p.m) {
+        if (p.status) p.status[s] = -4;  // GARAGE_EC_E_UNRECOVERABLE
+        return;
+    }
+    if (p.status) p.status[s] = 0;
+    if (absent || p.mismatch[s]) {
+        const uint32_t q = atomicAdd(p.count, 1u);
+        p.list[q] = s;
+        p.err_mask[q] = 0;
+        p.bad[q] = 0;
+    }
+}
+
+struct GfSmem {
+    uint8_t exp[512];
+    uint8_t log[256];
+};
+__device__ __forceinline__ uint32_t gf_mul_s(const GfSmem &g, uint32_t a, uint32_t b)
+{
+    return (a && b) ? g.exp[g.log[a] + g.log[b]] : 0u;
+}
+// a * alpha^lb, lb in [0, 255]
+__device__ __forceinline__ uint32_t gf_mul_l(const GfSmem &g, uint32_t a, uint32_t lb)
+{
+    return a ? g.exp[g.log[a] + lb] : 0u;
+}
+
+// Errors-and-erasures decoding of one byte column from its m GRS syndromes S (S_l = sum_r y_r v_r X_r^l,
+// erased y_r taken as 0) and the erasure locator gam = prod_{r in E} (1 + X_r x) of degree e:
+// Forney syndromes -> Berlekamp-Massey -> errata locator psi = lambda * gam and evaluator
+// omg = S * psi mod x^M.  Returns L = deg lambda, or -1 if 2L > m - e (more errors than t).
+// Every index is a compile-time constant, so the polynomials stay in registers.
+template <int M>
+__device__ __forceinline__ int correct_decode(const GfSmem &g, const uint32_t (&S)[M], const uint32_t (&gam)[M + 1], int e,
+                                              uint32_t (&psi)[M + 1], uint32_t (&omg)[M])
+{
+    uint32_t F[M];
+#pragma unroll
+    for (int i = 0; i < M; i++) {
+        uint32_t v = 0;
+#pragma unroll
+        for (int j = 0; j <= i; j++) v ^= gf_mul_s(g, S[j], gam[i - j]);
+        F[i] = v;
+    }
+    // Forney syndromes F[e .. M) moved down to F[0 .. M-e)
+#pragma unroll
+    for (int q = 0; q < M; q++) {
+        if (q < e) {
+#pragma unroll
+            for (int i = 0; i + 1 < M; i++) F[i] = F[i + 1];
+            F[M - 1] = 0;
+        }
+    }
+    const int N = M - e;
+    uint32_t C[M + 1], B[M + 1];  // B = x^shift * (previous connection polynomial)
+#pragma unroll
+    for (int i = 0; i <= M; i++) {
+        C[i] = i == 0 ? 1u : 0u;
+        B[i] = i == 1 ? 1u : 0u;
+    }
+    int L = 0;
+    uint32_t b = 1;
+#pragma unroll
+    for (int i = 0; i < M; i++) {
+        if (i < N) {
+            uint32_t d = F[i];
+#pragma unroll
+            for (int j = 1; j <= i; j++) d ^= gf_mul_s(g, C[j], F[i - j]);
+            if (d) {
+                const uint32_t lc = (uint32_t)g.log[d] + 255u - g.log[b];  // log(d / b), < 510
+                uint32_t T[M + 1];
+#pragma unroll
+                for (int j = 0; j <= M; j++) T[j] = C[j] ^ (B[j] ? g.exp[g.log[B[j]] + (lc % 255u)] : 0u);
+                if (2 * L <= i) {
+#pragma unroll
+                    for (int j = 0; j <= M; j++) B[j] = C[j];
+                    L = i + 1 - L;
+                    b = d;
+                }
+#pragma unroll
+                for (int j = 0; j <= M; j++) C[j] = T[j];
+            }
+#pragma unroll
+            for (int j = M; j > 0; j--) B[j] = B[j - 1];
+            B[0] = 0;
+        }
+    }
+    if (2 * L > N) return -1;
+#pragma unroll
+    for (int i = 0; i <= M; i++) {
+        uint32_t v = 0;
+#pragma unroll
+        for (int j = 0; j <= i; j++) v ^= gf_mul_s(g, C[j], gam[i - j]);
+        psi[i] = v;
+    }
+#pragma unroll
+    for (int i = 0; i < M; i++) {
+        uint32_t v = 0;
+#pragma unroll
+        for (int j = 0; j <= i; j++) v ^= gf_mul_s(g, S[j], psi[i - j]);
+        omg[i] = v;
+    }
+    return L;
+}
+
+// errata value at position r (log X_r = lx, log v_r = lv): psi(1/X_r) == 0 marks an errata position;
+// value y_r xor c_r = X_r omg(1/X_r) / (v_r psi'(1/X_r)).  Returns false where psi has no simple root.
+template <int M>
+__device__ __forceinline__ bool correct_value(const GfSmem &g, const uint32_t (&psi)[M + 1], const uint32_t (&omg)[M], uint32_t lx,
+                                              uint32_t lv, bool &errata, uint32_t &val)
+{
+    const uint32_t li = lx ? 255u - lx : 0u;  // log (1/X_r)
+    uint32_t ps = psi[M];
+#pragma unroll
+    for (int i = M - 1; i >= 0; i--) ps = gf_mul_l(g, ps, li) ^ psi[i];
+    errata = ps == 0;
+    val = 0;
+    if (!errata) return true;
+    uint32_t om = omg[M - 1];
+#pragma unroll
+    for (int i = M - 2; i >= 0; i--) om = gf_mul_l(g, om, li) ^ omg[i];
+    // psi'(x) = sum over odd i of psi[i] x^(i-1) (characteristic 2)
+    uint32_t dp = 0;
+#pragma unroll
+    for (int i = M - (M % 2 == 0 ? 1 : 0); i >= 1; i -= 2) dp = gf_mul_l(g, gf_mul_l(g, dp, li), li) ^ psi[i];
+    if (!dp) return false;
+    if (om) val = g.exp[(g.log[om] + lx + 2u * 255u - g.log[dp] - lv) % 255u];
+    return true;
+}
+
+// per work item: presence mask, erasure count and erasure locator of the stripe, staged by warp 0
+struct CorrectStripe {
+    unsigned long long pm;
+    uint32_t s, len, e, pad;
+    uint32_t gam[kMaxM + 1];
+};
+
+template <int M>
+__device__ __forceinline__ void correct_stage_stripe(const CorrectParams &p, const GfSmem &g, uint32_t s, CorrectStripe &cs)
+{
+    const uint32_t tid = threadIdx.x, tot = p.k + M;
+    if (tid >= 32) return;
+    const bool p0 = tid < tot && (!p.present || p.present[(size_t)s * tot + tid]);
+    const bool p1 = tid + 32 < tot && (!p.present || p.present[(size_t)s * tot + tid + 32]);
+    const unsigned long long pm =
+        (unsigned long long)__ballot_sync(0xffffffffu, p0) | ((unsigned long long)__ballot_sync(0xffffffffu, p1) << 32);
+    if (tid != 0) return;
+    cs.pm = pm;
+    cs.s = s;
+    cs.len = p.shard_len ? p.shard_len[s] : p.stride;
+    cs.e = tot - (uint32_t)__popcll(pm);
+    uint32_t gam[kMaxM + 1] = {1};
+    for (uint32_t r = 0; r < tot; r++) {
+        if ((pm >> r) & 1) continue;
+        for (int j = kMaxM; j > 0; j--) gam[j] ^= gf_mul_l(g, gam[j - 1], p.logx[r]);  // gam *= (1 + X_r x)
+    }
+    for (int j = 0; j <= kMaxM; j++) cs.gam[j] = gam[j];
+}
+
+// syndromes of byte column x of the stripe (x < len); absent shards count as zero
+template <int M>
+__device__ __forceinline__ void correct_syndromes(const CorrectParams &p, const GfSmem &g, const uint8_t *s_logh,
+                                                  const CorrectStripe &cs, uint32_t x, uint32_t (&S)[M])
+{
+    const uint32_t tot = p.k + M;
+    const uint8_t *col = p.shards + (size_t)cs.s * tot * p.stride + x;
+#pragma unroll
+    for (int l = 0; l < M; l++) S[l] = 0;
+#pragma unroll 2
+    for (uint32_t r = 0; r < tot; r++) {
+        if (!((cs.pm >> r) & 1)) continue;
+        const uint32_t y = __ldg(col + (size_t)r * p.stride);
+        if (!y) continue;
+        const uint32_t ly = g.log[y];
+#pragma unroll
+        for (int l = 0; l < M; l++) S[l] ^= g.exp[ly + s_logh[l * (kMaxK + kMaxM) + r]];
+    }
+}
+
+template <int M>
+__device__ __forceinline__ void correct_setup(const CorrectParams &p, GfSmem &g, uint8_t *s_logh)
+{
+    stage_gf_tables(reinterpret_cast<uint8_t *>(&g));
+    const uint32_t tot = p.k + M;
+    for (uint32_t i = threadIdx.x; i < M * tot; i += blockDim.x) {
+        const uint32_t l = i / tot, r = i - l * tot;
+        s_logh[l * (kMaxK + kMaxM) + r] = (uint8_t)((p.logv[r] + l * (uint32_t)p.logx[r]) % 255u);  // log(v_r X_r^l)
+    }
+}
+
+template <int M>
+__global__ void __launch_bounds__(kCorrectThreads) rs_correct_scan_kernel(const __grid_constant__ CorrectParams p)
+{
+    __shared__ __align__(16) GfSmem g;
+    __shared__ uint8_t s_logh[M * (kMaxK + kMaxM)];
+    __shared__ CorrectStripe cs;
+    correct_setup<M>(p, g, s_logh);
+    const uint32_t tid = threadIdx.x, lane = tid & 31, tot = p.k + M;
+    const unsigned long long total = (unsigned long long)*p.count * p.items_per_stripe;
+    for (unsigned long long item = blockIdx.x; item < total; item += gridDim.x) {
+        const uint32_t q = (uint32_t)(item / p.items_per_stripe), c = (uint32_t)(item - (unsigned long long)q * p.items_per_stripe);
+        __syncthreads();  // tables staged / previous item done with `cs`
+        correct_stage_stripe<M>(p, g, p.list[q], cs);
+        __syncthreads();
+        const uint32_t x = c * kCorrectThreads + tid;
+        unsigned long long errs = 0;
+        bool fail = false;
+        if (x < cs.len) {
+            uint32_t S[M];
+            correct_syndromes<M>(p, g, s_logh, cs, x, S);
+            uint32_t any = 0;
+#pragma unroll
+            for (int l = 0; l < M; l++) any |= S[l];
+            if (any) {  // clean columns (all-zero syndromes) of a listed stripe need nothing more
+                uint32_t gam[M + 1], psi[M + 1], omg[M];
+#pragma unroll
+                for (int j = 0; j <= M; j++) gam[j] = cs.gam[j];
+                const int L = correct_decode<M>(g, S, gam, (int)cs.e, psi, omg);
+                if (L < 0) {
+                    fail = true;
+                } else {
+                    // L distinct roots among the present positions, simple errata roots, and the errata pattern
+                    // must reproduce the syndromes: then y minus the pattern is the codeword within radius t
+                    uint32_t chk[M];
+#pragma unroll
+                    for (int l = 0; l < M; l++) chk[l] = 0;
+                    int roots = 0;
+                    for (uint32_t r = 0; r < tot && !fail; r++) {
+                        bool errata;
+                        uint32_t val;
+                        if (!correct_value<M>(g, psi, omg, p.logx[r], p.logv[r], errata, val)) fail = true;
+                        if (!errata) continue;
+                        const bool erased = !((cs.pm >> r) & 1);
+                        if (!erased) {
+                            roots++;
+                            if (val) errs |= 1ull << r;
+                        }
+                        if (val) {
+                            const uint32_t lv = g.log[val];
+#pragma unroll
+                            for (int l = 0; l < M; l++) chk[l] ^= g.exp[lv + s_logh[l * (kMaxK + kMaxM) + r]];
+                        }
+                    }
+                    if (roots != L) fail = true;
+#pragma unroll
+                    for (int l = 0; l < M; l++) fail |= chk[l] != S[l];
+                }
+            }
+        }
+        const uint32_t lo = __reduce_or_sync(0xffffffffu, (uint32_t)errs);
+        const uint32_t hi = __reduce_or_sync(0xffffffffu, (uint32_t)(errs >> 32));
+        const bool wfail = __any_sync(0xffffffffu, fail);
+        if (lane == 0) {
+            if (lo | hi) atomicOr(p.err_mask + q, ((unsigned long long)hi << 32) | lo);
+            if (wfail) atomicOr(p.bad + q, 1u);
+        }
+    }
+}
+
+template <int M>
+__global__ void __launch_bounds__(kCorrectThreads) rs_correct_apply_kernel(const __grid_constant__ CorrectParams p)
+{
+    __shared__ __align__(16) GfSmem g;
+    __shared__ uint8_t s_logh[M * (kMaxK + kMaxM)];
+    __shared__ CorrectStripe cs;
+    correct_setup<M>(p, g, s_logh);
+    const uint32_t tid = threadIdx.x, tot = p.k + M;
+    const unsigned long long total = (unsigned long long)*p.count * p.items_per_stripe;
+    for (unsigned long long item = blockIdx.x; item < total; item += gridDim.x) {
+        const uint32_t q = (uint32_t)(item / p.items_per_stripe), c = (uint32_t)(item - (unsigned long long)q * p.items_per_stripe);
+        __syncthreads();
+        correct_stage_stripe<M>(p, g, p.list[q], cs);
+        __syncthreads();
+        const uint32_t s = cs.s;
+        if (p.bad[q]) {  // uniform over the block: nothing of this stripe is written
+            if (c == 0 && tid == 0 && p.status) p.status[s] = -7;  // GARAGE_EC_E_UNCORRECTABLE
+            continue;
+        }
+        const unsigned long long errs = p.err_mask[q], absent = ~cs.pm & ((tot >= 64 ? 0ull : 1ull << tot) - 1ull);
+        if (c == 0 && p.fixed && tid < tot && ((errs >> tid) & 1)) p.fixed[(size_t)s * tot + tid] = 1;
+        const unsigned long long wr = errs | absent;  // shards to write
+        const uint32_t x = c * kCorrectThreads + tid;
+        if (!wr || x >= ((cs.len + 15u) & ~15u)) continue;
+        uint8_t *col = p.shards + (size_t)s * tot * p.stride + x;
+        if (x >= cs.len) {  // output padding
+            for (unsigned long long w = wr; w; w &= w - 1) col[(size_t)(__ffsll((long long)w) - 1) * p.stride] = 0;
+            continue;
+        }
+        uint32_t S[M];
+        correct_syndromes<M>(p, g, s_logh, cs, x, S);
+        uint32_t any = 0;
+#pragma unroll
+        for (int l = 0; l < M; l++) any |= S[l];
+        uint32_t gam[M + 1], psi[M + 1], omg[M];
+        if (any) {
+#pragma unroll
+            for (int j = 0; j <= M; j++) gam[j] = cs.gam[j];
+            correct_decode<M>(g, S, gam, (int)cs.e, psi, omg);  // succeeded in the scan pass
+        }
+        for (unsigned long long w = wr; w; w &= w - 1) {
+            const uint32_t r = (uint32_t)(__ffsll((long long)w) - 1);
+            const bool erased = (absent >> r) & 1;
+            uint32_t val = 0;
+            if (any) {
+                bool errata;
+                correct_value<M>(g, psi, omg, p.logx[r], p.logv[r], errata, val);
+            }
+            uint8_t *dst = col + (size_t)r * p.stride;
+            if (erased) *dst = (uint8_t)val;
+            else if (val) *dst = (uint8_t)(*dst ^ val);
+        }
+    }
+}
+
 }  // namespace garage_ec

@@ -58,6 +58,7 @@ extern "C" {
 #define GARAGE_EC_E_UNRECOVERABLE (-4) /* >= 1 stripe had < k shards; see status[] */
 #define GARAGE_EC_E_NODEVICE (-5)      /* no CUDA device / wrong architecture */
 #define GARAGE_EC_E_ALIGN (-6)         /* pointer or stride alignment violated */
+#define GARAGE_EC_E_UNCORRECTABLE (-7) /* >= 1 stripe had a column with more errors than t; see status[] */
 
 /* matrix kinds */
 #define GARAGE_EC_VANDERMONDE 0 /* systematic Vandermonde (default), G = V * inv(V[0..k)) */
@@ -135,6 +136,35 @@ int garage_ec_reconstruct_stripes(garage_ec_ctx *ctx, uint8_t *const *stripes, c
 int garage_ec_verify(garage_ec_ctx *ctx, const uint8_t *shards, uint32_t *mismatch,
                      const uint32_t *shard_len, size_t stride, size_t n_stripes, int mem_kind,
                      void *cuda_stream);
+
+/* ---- CORRECT (error-locating decode) -- call site: the DataBlock::verify failure on GET,
+ * src/block/block.rs:69-83 (the block's content hash does not match although every shard passed its
+ * own tag: a stale shard, a bad resync, bytes corrupted before they were tagged).  Finds and repairs
+ * shards that are present but WRONG, from the parity alone (normative definition: DESIGN.md section 2).
+ * Per stripe: e = number of absent shards, t = floor((m - e) / 2).
+ *   e > m     status = GARAGE_EC_E_UNRECOVERABLE, stripe untouched;
+ *   otherwise every byte column is decoded to the unique codeword that agrees with the received bytes
+ *             at all present positions but at most t.  If every column decodes, the codeword is written
+ *             into every absent shard and every present shard that differs from it (fixed[s*(k+m)+i] = 1
+ *             for those), status = 0, output padding [shard_len, roundup16) written as zero.  If some
+ *             column has no such codeword: status = GARAGE_EC_E_UNCORRECTABLE and NOTHING of the stripe
+ *             is written (fixed stays 0) -- callers fall back to per-shard tags or a leave-one-out search.
+ *   e = m     t = 0: a plain reconstruct, nothing is checked.
+ * A column with more than t errors can still land within distance t of another codeword (probability
+ * sum_{j<=t} C(k+m, j) 255^j / 256^m per column: ~0.14 % for RS(10,4), 2.3 % for RS(4,2)); the block's
+ * content hash or the shard tags stay the final check.
+ *   shards  : n * (k+m) * stride bytes, same layout / alignment / geometry rules as RECONSTRUCT
+ *   present : n * (k+m) bytes in {0,1}, NULL = all present
+ *   status  : n int32: 0, GARAGE_EC_E_UNRECOVERABLE or GARAGE_EC_E_UNCORRECTABLE
+ *   fixed   : NULL or n * (k+m) bytes
+ * HOST calls return GARAGE_EC_E_UNRECOVERABLE if any stripe was, else GARAGE_EC_E_UNCORRECTABLE if any
+ * stripe was, else 0; they upload the present shards and download only the rebuilt or fixed ones.
+ * DEVICE calls only fill status[] and never synchronise with the host (graph-capturable).
+ * The matrix must be a generalized RS code with evaluation points 0..k+m-1 (both built-in kinds are; so is
+ * garage_ec_create_with_matrix given a built-in matrix); for any other matrix this returns GARAGE_EC_E_INVALID. */
+int garage_ec_correct(garage_ec_ctx *ctx, uint8_t *shards, const uint8_t *present, int32_t *status,
+                      uint8_t *fixed, const uint32_t *shard_len, size_t stride, size_t n_stripes,
+                      int mem_kind, void *cuda_stream);
 
 /* ---- PER-SHARD INTEGRITY (SURVEY.md section 8 row f2) -- call sites: DataBlock::verify,
  * src/block/block.rs:69-83 (Plain => blake2sum(data) == hash) and read_block_from,

@@ -81,6 +81,33 @@ impl ErasureCoder {
         Ok(())
     }
 
+    /// GET whose block failed DataBlock::verify (src/block/block.rs:69-83) although every shard passed its
+    /// own tag: locate and repair the wrong shards of ONE stripe from the parity alone.  `shards[i]` is
+    /// Some(bytes) for every shard that arrived; on success the absent ones are filled in, the wrong ones
+    /// rewritten, and the indices of the rewritten shards are returned (quarantine them, queue resync).
+    /// Err(CorruptData) when some column has more wrong shards than the parity can locate: fall back to
+    /// the tags / a leave-one-out search.  The block hash stays the final check.
+    pub fn correct(&self, hash: &Hash, block_len: usize, shards: &mut [Option<Vec<u8>>]) -> Result<Vec<usize>, Error> {
+        let tot = self.k + self.m;
+        let l = self.shard_len(block_len);
+        let stride = unsafe { sys::garage_ec_stride_for(l as u32) };
+        let mut buf = vec![0u8; tot * stride];
+        let mut present = vec![0u8; tot];
+        for (i, s) in shards.iter().enumerate() {
+            if let Some(s) = s { buf[i * stride..i * stride + l].copy_from_slice(&s[..l]); present[i] = 1; }
+        }
+        let (mut status, mut fixed, lens) = ([0i32; 1], vec![0u8; tot], [l as u32; 1]);
+        let rc = unsafe { sys::garage_ec_correct(self.ctx, buf.as_mut_ptr(), present.as_ptr(), status.as_mut_ptr(),
+                          fixed.as_mut_ptr(), lens.as_ptr(), stride, 1, sys::GARAGE_EC_MEM_HOST, std::ptr::null_mut()) };
+        if rc == sys::GARAGE_EC_E_UNRECOVERABLE { return Err(Error::MissingBlock(*hash)); }
+        if rc == sys::GARAGE_EC_E_UNCORRECTABLE { return Err(Error::CorruptData(*hash)); }
+        check(self.ctx, rc)?;
+        for i in 0..tot {
+            if present[i] == 0 || fixed[i] != 0 { shards[i] = Some(buf[i * stride..i * stride + l].to_vec()); }
+        }
+        Ok((0..tot).filter(|&i| fixed[i] != 0).collect())
+    }
+
     /// Scrub: bit i of the result set = stored parity row i disagrees with the data shards.
     pub fn verify(&self, shards_layout: &[u8], shard_len: &[u32], stride: usize) -> Result<Vec<u32>, Error> {
         let n = shard_len.len();

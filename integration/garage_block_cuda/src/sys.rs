@@ -13,6 +13,7 @@ pub const GARAGE_EC_E_NOMEM: c_int = -3;
 pub const GARAGE_EC_E_UNRECOVERABLE: c_int = -4;
 pub const GARAGE_EC_E_NODEVICE: c_int = -5;
 pub const GARAGE_EC_E_ALIGN: c_int = -6;
+pub const GARAGE_EC_E_UNCORRECTABLE: c_int = -7;
 pub const GARAGE_EC_VANDERMONDE: c_int = 0;
 pub const GARAGE_EC_CAUCHY: c_int = 1;
 pub const GARAGE_EC_MEM_HOST: c_int = 0;
@@ -40,6 +41,9 @@ extern "C" {
                             n_stripes: usize, mem_kind: c_int, cuda_stream: *mut c_void) -> c_int;
     pub fn garage_ec_verify(ctx: *mut garage_ec_ctx, shards: *const u8, mismatch: *mut u32,
                             shard_len: *const u32, stride: usize, n_stripes: usize,
+                            mem_kind: c_int, cuda_stream: *mut c_void) -> c_int;
+    pub fn garage_ec_correct(ctx: *mut garage_ec_ctx, shards: *mut u8, present: *const u8, status: *mut i32,
+                            fixed: *mut u8, shard_len: *const u32, stride: usize, n_stripes: usize,
                             mem_kind: c_int, cuda_stream: *mut c_void) -> c_int;
     pub fn garage_ec_encode_blocks(ctx: *mut garage_ec_ctx, blocks: *const *const u8,
                             block_len: *const u32, n_blocks: usize, parity_out: *mut u8,
